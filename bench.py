@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- solver-update throughput of the DPM-Solver hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4] [--dump-outputs DIR]
 
 One "step" = one full DPM_Solver.sample() over one batch of synthetic input (BASELINE.json
 configs[1]: DPM-Solver++ 2M, 20 solver updates, synthetic eps, bf16 latents [4096,4,64,64] per GPU).
@@ -21,6 +21,11 @@ metric = solver-update GElem/s = elements(x) * updates / seconds, whole job over
   workloads : (default N=1 run) the other single-GPU BASELINE configs, c3 and c4, each with value / roofline / clocks
   parity    : outside the timed region, a batch slice of the run's own output is compared with the UNMODIFIED
               reference (oracle/_ref, CPU fp32) on the same inputs -> config.parity_checked
+
+--dump-outputs DIR writes what the last timed sample() of the headline workload returned (rank 0), as float32:
+DIR/x_0.npy holds DUMP_ROWS samples of the batch, rows picked by a fixed seed. The inputs are seeded and the
+synthetic network's bank rotation depends only on --steps / --warmup, so two builds of the project run with the same
+arguments can be compared output for output.
 
 --impl reference runs the UNMODIFIED reference (oracle/_ref: /root/reference/dpm_solver_pytorch.py byte-compiled by
 oracle/build_ref.py, shipped to the box) on the host cores; the oracle port is only the fallback when that
@@ -644,8 +649,22 @@ def shard_parity(ctx, w):
     return bool(flag.item())
 
 
-def measure(ctx, args, name, w, steps, warmup, with_e2e=True):
-    """Time one workload on this process's GPU; returns the dict of a bench line (rank 0) or None."""
+DUMP_ROWS = 512             # c2 / c3: [512, 4, 64, 64] float32 = 32 MB
+DUMP_MAX_ELEMS = 8 << 20    # c4: 42 rows of [3, 256, 256]
+
+
+def dump_outputs(y, out_dir):
+    """A fixed, seeded sample of rows of the output `y` (at most DUMP_MAX_ELEMS elements) -> out_dir/x_0.npy."""
+    per = int(np.prod(y.shape[1:]))
+    n = max(1, min(y.shape[0], DUMP_ROWS, DUMP_MAX_ELEMS // per))
+    rows = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x_0.npy"), y[rows.to(y.device)].float().cpu().numpy())
+
+
+def measure(ctx, args, name, w, steps, warmup, with_e2e=True, dump_dir=None):
+    """Time one workload on this process's GPU; returns the dict of a bench line (rank 0) or None. With `dump_dir`,
+    rank 0 writes a sample of the last timed step's output there (dump_outputs)."""
     be, dev, world, rank = ctx.be, ctx.dev, ctx.world, ctx.rank
     dt = DT[w["dtype"]]
     shape = tuple(w["shape"])
@@ -673,6 +692,8 @@ def measure(ctx, args, name, w, steps, warmup, with_e2e=True):
         ctx.barrier()
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
     gpu_launches = be.launch_count() - launches0
+    if dump_dir is not None and rank == 0:
+        dump_outputs(y, dump_dir)
     # ---- instrumented pass: the same K steps again with CUDA events around every library launch (per-kernel
     # durations for the roofline / kernels breakdown); its whole-pass time is reported as ms_per_step_instrumented
     be.recording, be.records = True, []
@@ -797,7 +818,7 @@ def measure(ctx, args, name, w, steps, warmup, with_e2e=True):
 
 def run_b200(args, w):
     ctx = Ctx(args)
-    out = measure(ctx, args, args.workload, w, args.steps, args.warmup)
+    out = measure(ctx, args, args.workload, w, args.steps, args.warmup, dump_dir=args.dump_outputs)
     if ctx.world > 1:
         ok = shard_parity(ctx, w)
         if ctx.rank == 0:
@@ -850,7 +871,11 @@ def main():
     ap.add_argument("--ctas", type=int, default=0)
     ap.add_argument("--no-extras", action="store_true", help="skip the c3/c4, kernel-alone and CPU-baseline legs")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the process to the GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's output to DIR/x_0.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -6,8 +6,11 @@ import numpy as np
 import pytest
 import torch
 
+import refstore as S
 from cases import exact_net, make_betas, seeded
 from helpers import product_schedule, rel_err
+
+REF = S.Store(__file__)
 
 CASES = [
     dict(name="ad23_eps_vp", schedule="vp_linear", algo="dpmsolver", order=3, t_end=1e-3, solver_type="dpmsolver"),
@@ -96,11 +99,7 @@ def test_device_controller_matches_reference(cuda_backend, chunk):
     import contextlib
     import io
     import dpm_solver_b200 as new
-    from oracle import ref_loader
     from test_random_configs_vs_reference import run_wide
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref not built")
-    ref = ref_loader.load("dpm_solver_pytorch")
 
     class OnGpu:        # run_wide() builds CPU tensors: move the product arm to the device
         NoiseScheduleVP = new.NoiseScheduleVP
@@ -116,18 +115,21 @@ def test_device_controller_matches_reference(cuda_backend, chunk):
 
     from unittest import mock
     seen_device = 0
-    for c in _adaptive_cfgs(10, 9000 + chunk):
+    def reference(c):
         with mock.patch("builtins.print") as pr:           # both print 'adaptive solver nfe', N (:1009)
-            yr, _, _ = run_wide(ref, c)
-        nfe_r = pr.call_args[0][-1]
-        if not torch.isfinite(yr).all():
+            yr, _, _ = run_wide(S.original(), c)
+        return S.sample(yr), pr.call_args[0][-1]
+
+    for i, c in enumerate(_adaptive_cfgs(10, 9000 + chunk)):
+        yr, nfe_r = REF(f"device_controller/{chunk}/{i}", lambda: reference(c))
+        if not S.all_finite(yr):
             continue
         before = cuda_backend.launch_count()
         with mock.patch("builtins.print") as pn:
             yn, _, _ = run_wide(OnGpu, c)
         seen_device += cuda_backend.launch_count() > before
         assert pn.call_args[0][-1] == nfe_r, ("NFE", c)
-        assert rel_err(yn.numpy(), yr.numpy()) <= 2e-4, c      # measured: 0 .. 5e-5 (profiles/r02_adaptive_probe.txt)
+        assert yr.rel_err(yn) <= 2e-4, c      # measured: 0 .. 5e-5 (profiles/r02_adaptive_probe.txt)
     assert seen_device
 
 

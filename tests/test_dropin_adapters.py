@@ -16,7 +16,8 @@ import torch
 import adapters as A
 from helpers import rel_err
 
-pytestmark = pytest.mark.skipif(not A.available(), reason="oracle/_ref not built and no reference tree")
+# the adapters are the original project's own example code, which is not part of this repository
+needs_adapters = pytest.mark.skipif(not A.available(), reason="the original project's example adapters are not available")
 
 EXECUTORS = ["numpy-executor", pytest.param("cuda", marks=pytest.mark.gpu)]
 
@@ -42,6 +43,7 @@ def _launches():
     return be.launch_count() if hasattr(be, "launch_count") else 0
 
 
+@needs_adapters
 @pytest.mark.parametrize("order,steps,method", [(2, 20, "multistep"), (3, 12, "multistep"), (2, 9, "singlestep")])
 @pytest.mark.parametrize("tables", ["host", "device"])
 def test_stable_diffusion_adapter_runs_unchanged(product_device, order, steps, method, tables):
@@ -91,6 +93,7 @@ def _sde_net(x, t):
     return 0.1 * x + ((t * 0.05) - 0.02).reshape(-1, 1, 1, 1)
 
 
+@needs_adapters
 @pytest.mark.parametrize("kw", [dict(), dict(denoise=True, steps=13), dict(algorithm_type="dpmsolver++", thresholding=True, order=2, steps=8),
                                 dict(skip_type="time_uniform", method="multistep", order=2, steps=12)])
 def test_score_sde_glue_runs_unchanged(product_device, kw):
@@ -108,6 +111,7 @@ def test_score_sde_glue_runs_unchanged(product_device, kw):
     np.testing.assert_array_equal(outs[1][0].numpy(), outs[0][0].numpy())
 
 
+@needs_adapters
 @pytest.mark.parametrize("kw", [dict(),                                                       # classifier guidance + thresholding, ++3M
                                 dict(cond_class=False, thresholding=False, sample_type="dpmsolver", order=2, method="singlestep"),
                                 dict(denoise=True, timesteps=10, order=2),

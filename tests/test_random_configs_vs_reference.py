@@ -1,29 +1,25 @@
-"""Randomised end-to-end parity against the UNMODIFIED reference (oracle/_ref).
+"""Randomised end-to-end parity against the UNMODIFIED reference (its results stored in tests/golden/reference/).
 
 Draws sampling configurations at random (schedule, algorithm, method, order, steps, skip type,
 solver type, parameterisation, CFG, thresholding, t_end, denoise_to_zero), runs the reference on CPU
 and the product's host logic on the numpy executor, and requires bit-identical outputs and an
 identical trace of network calls. Complements the fixed golden cases of tests/golden/."""
-import os
 import random
-import sys
 import warnings
 
-import numpy as np
 import pytest
 import torch
 
-from oracle import ref_loader  # noqa: E402
+import refstore as S
+from cases import exact_net, make_betas, seeded
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="oracle/_ref not built and no reference tree")
-
-from cases import exact_net, make_betas, seeded  # noqa: E402
+REF = S.Store(__file__)
 
 
 def reference_module():
-    """The unmodified reference (oracle/_ref bytecode of /root/reference/dpm_solver_pytorch.py)."""
+    """The unmodified reference dpm_solver_pytorch.py (only run while recording tests/golden/reference/)."""
     warnings.filterwarnings("ignore")
-    return ref_loader.load("dpm_solver_pytorch")
+    return S.original("dpm_solver_pytorch")
 
 
 def draw(rng):
@@ -69,26 +65,30 @@ def run(mod_ns, mod_wrap, mod_solver, c):
 @pytest.mark.parametrize("chunk", range(6))
 def test_random_configurations_bit_exact(oracle_backend, chunk):
     import dpm_solver_b200 as new
-    ref = reference_module()
     rng = random.Random(1000 + chunk)
     done = 0
+    i = 0
     while done < 12:
         c = draw(rng)
+        i += 1
         try:
-            yr, ir, cr = run(ref.NoiseScheduleVP, ref.model_wrapper, ref.DPM_Solver, c)
+            yr, ir, cr = REF(f"bit_exact/{chunk}/{i}", lambda: run_reference(c))
         except Exception as e:   # configurations the reference itself rejects must be rejected the same way
             with pytest.raises(type(e)):
                 run(new.NoiseScheduleVP, new.model_wrapper, new.DPM_Solver, c)
             continue
-        if not torch.isfinite(yr).all():
+        if not S.all_finite(yr):
             continue
         yn, in_, cn = run(new.NoiseScheduleVP, new.model_wrapper, new.DPM_Solver, c)
-        assert cn == cr, c
-        np.testing.assert_array_equal(yn.numpy(), yr.numpy(), err_msg=str(c))
-        assert len(in_) == len(ir), c
-        for a, b in zip(in_, ir):
-            np.testing.assert_array_equal(a.numpy(), b.numpy(), err_msg=str(c))
+        S.assert_same(cn, cr, c)
+        S.assert_same(yn, yr, c)
+        S.assert_same(in_, ir, c)
         done += 1
+
+
+def run_reference(c):
+    ref = reference_module()
+    return run(ref.NoiseScheduleVP, ref.model_wrapper, ref.DPM_Solver, c)
 
 
 def draw_wide(rng):
@@ -142,28 +142,32 @@ def test_random_wide_configurations(oracle_backend, chunk):
     same number of times and agree within the reduction-order tolerance of its error estimate
     (tests/test_adaptive.py; 596 random adaptive runs: 500 bit-identical, worst 1.9e-4 relative)."""
     import dpm_solver_b200 as new
-    ref = reference_module()
+
+    def reference(c):
+        y, inter, calls = run_wide(reference_module(), c)
+        if c["method"] == "adaptive":       # compared within a tolerance, by the number of network calls
+            return S.sample(y), inter, len(calls)
+        return y, inter, calls
+
     rng = random.Random(5000 + chunk)
-    for _ in range(20):
+    for i in range(20):
         c = draw_wide(rng)
         try:
-            yr, ir, cr = run_wide(ref, c)
+            yr, ir, cr = REF(f"wide/{chunk}/{i}", lambda: reference(c))
         except Exception as e:
             with pytest.raises(type(e)):
                 run_wide(new, c)
             continue
-        if not torch.isfinite(yr).all():
+        if not S.all_finite(yr):
             continue
         yn, in_, cn = run_wide(new, c)
         if c["method"] == "adaptive":
-            assert len(cn) == len(cr), c
-            assert float((yn - yr).abs().max()) <= 1e-3 * float(yr.abs().max()), c
+            assert len(cn) == cr, c
+            assert yr.rel_err(yn) <= 1e-3, c
             continue
-        assert cn == cr, c
-        np.testing.assert_array_equal(yn.numpy(), yr.numpy(), err_msg=str(c))
-        assert len(in_) == len(ir), c
-        for a, b in zip(in_, ir):
-            np.testing.assert_array_equal(a.numpy(), b.numpy(), err_msg=str(c))
+        S.assert_same(cn, cr, c)
+        S.assert_same(yn, yr, c)
+        S.assert_same(in_, ir, c)
 
 
 @pytest.mark.parametrize("dt", [torch.bfloat16, torch.float16], ids=["bf16", "f16"])
@@ -173,39 +177,41 @@ def test_16bit_inputs_follow_the_reference_promotion(oracle_backend, dt):
     the widened values -- dtype trace and samples bit-identical to the reference. (16-bit CFG outputs and
     the 0-dim coefficients of the 'linear' schedule are documented deviations, DESIGN.md section 2.)"""
     import dpm_solver_b200 as new
-    ref = reference_module()
+
+    def arm(mod, c):
+        _, betas = make_betas(c["schedule"])
+        ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
+        calls = []
+
+        def net(xx, tt, *cond):
+            calls.append((float(tt[0]), tuple(xx.shape), xx.dtype))
+            return exact_net(xx.float(), tt).to(xx.dtype)
+        if c["cfg"] is not None:
+            fn = mod.model_wrapper(net, ns, model_type=c["model_type"], guidance_type="classifier-free",
+                                   condition=torch.ones(c["B"], 1), unconditional_condition=torch.zeros(c["B"], 1),
+                                   guidance_scale=c["cfg"])
+        else:
+            fn = mod.model_wrapper(net, ns, model_type=c["model_type"])
+        s = mod.DPM_Solver(fn, ns, algorithm_type=c["algo"], correcting_x0_fn="dynamic_thresholding" if c["thresholding"] else None)
+        x = (seeded((c["B"],) + c["shape"], c["seed"]) * c["scale"]).to(dt)
+        y = s.sample(x, steps=c["steps"], order=c["order"], skip_type=c["skip_type"], method=c["method"],
+                     lower_order_final=c["lower_order_final"], denoise_to_zero=c["denoise_to_zero"],
+                     solver_type=c["solver_type"], t_end=c["t_end"], t_start=c["t_start"])
+        return y, calls
+
     rng = random.Random(77)
-    done = 0
+    done = i = 0
     while done < 25:
         c = draw_wide(rng)
         if c["method"] == "adaptive" or c["schedule"] == "vp_linear" or c["cfg"] not in (None, 1.0):
             continue
-        outs = []
-        for mod in (ref, new):
-            _, betas = make_betas(c["schedule"])
-            ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
-            calls = []
-
-            def net(xx, tt, *cond):
-                calls.append((float(tt[0]), tuple(xx.shape), xx.dtype))
-                return exact_net(xx.float(), tt).to(xx.dtype)
-            if c["cfg"] is not None:
-                fn = mod.model_wrapper(net, ns, model_type=c["model_type"], guidance_type="classifier-free",
-                                       condition=torch.ones(c["B"], 1), unconditional_condition=torch.zeros(c["B"], 1),
-                                       guidance_scale=c["cfg"])
-            else:
-                fn = mod.model_wrapper(net, ns, model_type=c["model_type"])
-            s = mod.DPM_Solver(fn, ns, algorithm_type=c["algo"], correcting_x0_fn="dynamic_thresholding" if c["thresholding"] else None)
-            x = (seeded((c["B"],) + c["shape"], c["seed"]) * c["scale"]).to(dt)
-            y = s.sample(x, steps=c["steps"], order=c["order"], skip_type=c["skip_type"], method=c["method"],
-                         lower_order_final=c["lower_order_final"], denoise_to_zero=c["denoise_to_zero"],
-                         solver_type=c["solver_type"], t_end=c["t_end"], t_start=c["t_start"])
-            outs.append((y, calls))
-        (yr, cr), (yn, cn) = outs
-        if not torch.isfinite(yr).all():
+        i += 1
+        yr, cr = REF(f"16bit_inputs/{dt}/{i}", lambda: arm(reference_module(), c))
+        if not S.all_finite(yr):
             continue
-        assert cn == cr, c
-        assert yn.dtype == yr.dtype and torch.equal(yn, yr), c
+        yn, cn = arm(new, c)
+        S.assert_same(cn, cr, c)
+        S.assert_same(yn, yr, c)
         done += 1
 
 
@@ -217,9 +223,33 @@ def test_reference_rounding_mode_is_bit_identical(oracle_backend, x_16bit):
     the option on, samples are bit-identical to the reference for every parameterisation, with and
     without CFG (scales that are not representable in bf16 included), fp32 or 16-bit x_T."""
     import dpm_solver_b200 as new
-    ref = reference_module()
+
+    def arm(mod, c, dt):
+        _, betas = make_betas(c["schedule"])
+        ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
+
+        def net(xx, tt, *cond):
+            o = exact_net(xx.float(), tt)
+            if cond:
+                o = o + 0.05 * cond[0].reshape(-1, 1, 1, 1)
+            return o.to(dt)
+        if c["cfg"] is not None:
+            fn = mod.model_wrapper(net, ns, model_type=c["model_type"], guidance_type="classifier-free",
+                                   condition=torch.ones(c["B"], 1), unconditional_condition=torch.zeros(c["B"], 1),
+                                   guidance_scale=c["cfg"])
+        else:
+            fn = mod.model_wrapper(net, ns, model_type=c["model_type"])
+        kw = dict(reference_rounding=True) if mod is new else {}
+        s = mod.DPM_Solver(fn, ns, algorithm_type=c["algo"],
+                           correcting_x0_fn="dynamic_thresholding" if c["thresholding"] else None, **kw)
+        x = seeded((c["B"],) + c["shape"], c["seed"]) * c["scale"]
+        y = s.sample(x.to(dt) if x_16bit else x, steps=c["steps"], order=c["order"], skip_type=c["skip_type"],
+                     method=c["method"], lower_order_final=c["lower_order_final"], denoise_to_zero=c["denoise_to_zero"],
+                     solver_type=c["solver_type"], t_end=c["t_end"], t_start=c["t_start"])
+        return y
+
     rng = random.Random(4242 + int(x_16bit))
-    done = 0
+    done = i = 0
     while done < 30:
         c = draw_wide(rng)
         if c["method"] == "adaptive" or c["schedule"] == "vp_linear":
@@ -227,34 +257,12 @@ def test_reference_rounding_mode_is_bit_identical(oracle_backend, x_16bit):
         dt = rng.choice([torch.bfloat16, torch.float16])
         if c["cfg"] not in (None, 1.0) and rng.random() < 0.5:
             c["cfg"] = rng.choice([3.7, 2.3, 9.1])
-        outs = []
-        for mod in (ref, new):
-            _, betas = make_betas(c["schedule"])
-            ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
-
-            def net(xx, tt, *cond):
-                o = exact_net(xx.float(), tt)
-                if cond:
-                    o = o + 0.05 * cond[0].reshape(-1, 1, 1, 1)
-                return o.to(dt)
-            if c["cfg"] is not None:
-                fn = mod.model_wrapper(net, ns, model_type=c["model_type"], guidance_type="classifier-free",
-                                       condition=torch.ones(c["B"], 1), unconditional_condition=torch.zeros(c["B"], 1),
-                                       guidance_scale=c["cfg"])
-            else:
-                fn = mod.model_wrapper(net, ns, model_type=c["model_type"])
-            kw = dict(reference_rounding=True) if mod is new else {}
-            s = mod.DPM_Solver(fn, ns, algorithm_type=c["algo"],
-                               correcting_x0_fn="dynamic_thresholding" if c["thresholding"] else None, **kw)
-            x = seeded((c["B"],) + c["shape"], c["seed"]) * c["scale"]
-            y = s.sample(x.to(dt) if x_16bit else x, steps=c["steps"], order=c["order"], skip_type=c["skip_type"],
-                         method=c["method"], lower_order_final=c["lower_order_final"], denoise_to_zero=c["denoise_to_zero"],
-                         solver_type=c["solver_type"], t_end=c["t_end"], t_start=c["t_start"])
-            outs.append(y)
-        yr, yn = outs
-        if not torch.isfinite(yr).all():
+        i += 1
+        yr = REF(f"reference_rounding/{x_16bit}/{i}", lambda: arm(reference_module(), c, dt))
+        if not S.all_finite(yr):
             continue
-        assert yn.dtype == yr.dtype and torch.equal(yn, yr), (c, dt)
+        yn = arm(new, c, dt)
+        S.assert_same(yn, yr, (c, dt))
         done += 1
 
 
@@ -263,7 +271,6 @@ def test_classifier_guidance_matches_reference(oracle_backend, model_type):
     """guidance_type='classifier' (:315-321): eps - s*sigma_t*grad_x log p(c|x); the guided-diffusion
     example drives the solver this way (runners/diffusion.py:611-628)."""
     import dpm_solver_b200 as new
-    ref = reference_module()
     kind, betas = make_betas("ddpm_linear")
     W = torch.randn(5, 3 * 8 * 8, generator=torch.Generator().manual_seed(0)) * 0.05
 
@@ -274,17 +281,18 @@ def test_classifier_guidance_matches_reference(oracle_backend, model_type):
 
     cond = torch.tensor([1, 3])
     x = seeded((2, 3, 8, 8), 11)
-    outs = []
-    for mod in (ref, new):
+    def arm(mod):
         ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
         fn = mod.model_wrapper(exact_net, ns, model_type=model_type, guidance_type="classifier", condition=cond,
                                guidance_scale=2.5, classifier_fn=classifier_fn)
         eps = fn(x, torch.full((2,), 0.6))
         s = mod.DPM_Solver(fn, ns, algorithm_type="dpmsolver++", correcting_x0_fn="dynamic_thresholding")
         y = s.sample(x, steps=8, order=2)
-        outs.append((eps, y))
-    np.testing.assert_array_equal(outs[1][0].numpy(), outs[0][0].numpy())
-    np.testing.assert_array_equal(outs[1][1].numpy(), outs[0][1].numpy())
+        return eps, y
+
+    want = REF(f"classifier_guidance/{model_type}", lambda: arm(reference_module()))
+    for a, b in zip(arm(new), want):
+        S.assert_same(a, b)
 
 
 @pytest.mark.parametrize("method,order,steps", [("multistep", 2, 12), ("multistep", 3, 9), ("singlestep", 3, 10), ("singlestep_fixed", 2, 8)])
@@ -293,14 +301,12 @@ def test_hooks_match_reference(oracle_backend, method, order, steps, cfg):
     """correcting_xt_fn (DiffEdit-style inpainting mask, :1180-1239) and a user correcting_x0_fn
     (:440-441) see the same arguments in the same order and produce bit-identical samples."""
     import dpm_solver_b200 as new
-    ref = reference_module()
     kind, betas = make_betas("sd")
     B = 2
     x = seeded((B, 3, 8, 8), 31)
     mask = (seeded((B, 3, 8, 8), 32) > 0).float()
     known = seeded((B, 3, 8, 8), 33)
-    outs = []
-    for mod in (ref, new):
+    def arm(mod):
         ns = mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
         log = []
 
@@ -318,23 +324,25 @@ def test_hooks_match_reference(oracle_backend, method, order, steps, cfg):
             fn = mod.model_wrapper(exact_net, ns)
         s = mod.DPM_Solver(fn, ns, algorithm_type="dpmsolver++", correcting_x0_fn=fix_x0, correcting_xt_fn=fix_xt)
         y, inter = s.sample(x, steps=steps, order=order, method=method, return_intermediate=True, denoise_to_zero=True)
-        outs.append((y, inter, log))
-    assert outs[0][2] == outs[1][2]
-    np.testing.assert_array_equal(outs[1][0].numpy(), outs[0][0].numpy())
-    for a, b in zip(outs[1][1], outs[0][1]):
-        np.testing.assert_array_equal(a.numpy(), b.numpy())
+        return y, inter, log
+
+    yr, ir, lr = REF(f"hooks/{method}/{order}/{steps}/{cfg}", lambda: arm(reference_module()))
+    yn, in_, ln = arm(new)
+    S.assert_same(ln, lr)
+    S.assert_same(yn, yr)
+    S.assert_same(in_, ir)
 
 
 @pytest.mark.parametrize("steps,order", [(2, 3), (1, 2), (1, 3)])
 def test_singlestep_fixed_with_fewer_steps_than_order(oracle_backend, steps, order):
     """K = steps // order = 0: the reference runs no outer step and returns x (plus the optional denoise tail)."""
     import dpm_solver_b200 as new
-    ref = reference_module()
     for d2z in (False, True):
         c = dict(schedule="sd", algo="dpmsolver++", method="singlestep_fixed", order=order, steps=steps, skip_type="time_uniform",
                  solver_type="dpmsolver", model_type="noise", cfg=None, lower_order_final=True, denoise_to_zero=d2z, t_end=None,
                  seed=5, thresholding=False)
-        yr, ir, cr = run(ref.NoiseScheduleVP, ref.model_wrapper, ref.DPM_Solver, c)
+        yr, ir, cr = REF(f"fewer_steps/{steps}/{order}/{d2z}", lambda: run_reference(c))
         yn, in_, cn = run(new.NoiseScheduleVP, new.model_wrapper, new.DPM_Solver, c)
-        assert cn == cr and len(in_) == len(ir)
-        np.testing.assert_array_equal(yn.numpy(), yr.numpy())
+        S.assert_same(cn, cr)
+        S.assert_same(in_, ir)
+        S.assert_same(yn, yr)

@@ -1,14 +1,16 @@
-"""Randomised parity of the DIRECTLY callable solver methods against the UNMODIFIED reference (build
-container only): every public update method, the order dispatchers, the model functions, add_noise and
+"""Randomised parity of the DIRECTLY callable solver methods against the UNMODIFIED reference (its results stored
+in tests/golden/reference/): every public update method, the order dispatchers, the model functions, add_noise and
 inverse, with random times, r1/r2, solver_type, parameterisation and thresholding. Bit-identical."""
 import random
 
-import numpy as np
 import pytest
 import torch
 
+import refstore as S
 from cases import exact_net, make_betas, seeded
-from test_random_configs_vs_reference import reference_module, pytestmark  # noqa: F401  (same skip rule)
+from test_random_configs_vs_reference import reference_module
+
+REF = S.Store(__file__)
 
 
 def mk(mod, c):
@@ -60,7 +62,6 @@ def one(mod, c):
 @pytest.mark.parametrize("chunk", range(4))
 def test_direct_api_bit_exact(oracle_backend, chunk):
     import dpm_solver_b200 as new
-    ref = reference_module()
     for seed in range(75 * chunk, 75 * (chunk + 1)):
         rng = random.Random(31000 + seed)
         c = dict(schedule=rng.choice(["sd", "ddpm_linear", "iddpm_cosine", "vp_linear"]), algo=rng.choice(["dpmsolver++", "dpmsolver"]),
@@ -73,17 +74,17 @@ def test_direct_api_bit_exact(oracle_backend, chunk):
         if c["r1"] is not None and c["r2"] is not None and c["r2"] <= c["r1"]:
             c["r2"] = min(0.95, c["r1"] + 0.2)
         try:
-            a = one(ref, c)
+            a = REF(f"direct/{seed}", lambda: one(reference_module(), c))
         except Exception as e:   # what the reference rejects must be rejected the same way
             with pytest.raises(type(e)):
                 one(new, c)
             continue
-        if not all(torch.isfinite(v).all() for v in a):
+        if not all(S.all_finite(v) for v in a):
             continue
         b = one(new, c)
         assert len(a) == len(b), c
         for u, v in zip(a, b):
-            np.testing.assert_array_equal(v.numpy(), u.numpy(), err_msg=str(c))
+            S.assert_same(v, u, c)
 
 
 @pytest.mark.parametrize("chunk", range(2))
@@ -91,7 +92,6 @@ def test_model_fn_with_per_sample_times(oracle_backend, chunk):
     """`model_fn(x, t_continuous)` called directly with a VECTOR of different times (the reference's wrapper
     accepts it for every parameterisation and guidance type, :282-330): bit-identical."""
     import dpm_solver_b200 as new
-    ref = reference_module()
     for seed in range(40 * chunk, 40 * (chunk + 1)):
         rng = random.Random(seed)
         sched = rng.choice(["sd", "ddpm_linear", "iddpm_cosine", "vp_linear"])
@@ -102,8 +102,7 @@ def test_model_fn_with_per_sample_times(oracle_backend, chunk):
         tt = (torch.full((B,), rng.uniform(0.01, 1.0)) if rng.random() < 0.3
               else torch.tensor([rng.uniform(0.01, 1.0) for _ in range(B)]))
         x = seeded((B, 3, 8, 8), seed)
-        outs = []
-        for mod in (ref, new):
+        def arm(mod):
             kind, betas = make_betas(sched)
             ns = mod.NoiseScheduleVP("linear") if kind == "linear" else mod.NoiseScheduleVP("discrete", betas=torch.from_numpy(betas))
             if g == "uncond":
@@ -117,6 +116,6 @@ def test_model_fn_with_per_sample_times(oracle_backend, chunk):
                     return -((xx - 0.1 * cond.reshape(-1, 1, 1, 1)) ** 2).flatten(1).sum(1) * 0.01 + 0 * t_in
                 fn = mod.model_wrapper(lambda xx, t: exact_net(xx, t), ns, model_type=mt, guidance_type="classifier",
                                        condition=torch.ones(B), guidance_scale=scale, classifier_fn=cls)
-            outs.append(fn(x, tt))
-        a, b = outs
-        assert a.dtype == b.dtype and a.shape == b.shape and torch.equal(a, b), (sched, mt, g, scale)
+            return fn(x, tt)
+        a = REF(f"model_fn/{seed}", lambda: arm(reference_module()))
+        S.assert_same(arm(new), a, (sched, mt, g, scale))
