@@ -70,6 +70,7 @@ PROTOTYPES = {
     "dpm_duplicate": (C.c_int, [_vp, _vp, _u64, _i, _vp]),
     "dpm_philox_policy": (C.c_int, [_u64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
     "dpm_add_noise_philox": (C.c_int, [_vp, _vp, _u64, _i, C.POINTER(C.c_float), C.POINTER(C.c_float), _u64, _u64, _i, _i, _vp]),
+    "dpm_sde_step": (C.c_int, [C.POINTER(StepDesc), _f, _vp, _u64, _u64, _vp]),
     "dpm_diffedit_corrector": (C.c_int, [_vp, _vp, _vp, _vp, _u64, _u64, _f, _f, _u64, _u64, _i, _vp]),
     "dpm_data_prediction": (C.c_int, [_vp, _vp, _vp, _f, _f, _vp, _u64, _u64, _i, _vp]),
     "dpm_dynamic_threshold_workspace": (C.c_size_t, [_u64, _u64]),

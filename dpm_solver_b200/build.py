@@ -25,10 +25,11 @@ OUT_DIR = PKG / "lib"
 BUILD_DIR = PKG / "build"
 LIB_NAME = "libdpmsolver_b200.so"
 
-SOURCES = ["capi.cu", "step_direct.cu", "step_tma.cu", "quantile.cu", "adaptive.cu", "adaptive_ctl.cu", "philox.cu"]
-# philox.cu embeds curand's Box-Muller, which must round exactly like the copy inside torch's randn kernel: it is
-# compiled with nvcc's default fma contraction and spells the reference's unfused chain with __fmul_rn/__fadd_rn
-FMAD_DEFAULT = {"philox.cu"}
+SOURCES = ["capi.cu", "step_direct.cu", "step_tma.cu", "quantile.cu", "adaptive.cu", "adaptive_ctl.cu", "philox.cu",
+           "step_sde.cu"]
+# philox.cu and step_sde.cu embed curand's Box-Muller, which must round exactly like the copy inside torch's randn
+# kernel: they are compiled with nvcc's default fma contraction and spell the unfused chains with __fmul_rn/__fadd_rn
+FMAD_DEFAULT = {"philox.cu", "step_sde.cu"}
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-fmad=false", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]

@@ -248,6 +248,27 @@ static int step_impl(const dpm_step_desc* d, cudaStream_t stream) {
   return finish(stream);
 }
 
+static int sde_step_impl(const dpm_step_desc* d, float cn, const float* noise, uint64_t seed, uint64_t offset,
+                         cudaStream_t stream) {
+  if (d == nullptr) { set_error("desc is NULL"); return DPM_ERR_ARG; }
+  if (d->n == 0) return DPM_OK;
+  if (d->form != DPM_FORM_LIN1 && d->form != DPM_FORM_DIFF2) {
+    set_error("dpm_sde_step serves DPM_FORM_LIN1 and DPM_FORM_DIFF2 only (form %d)", d->form);
+    return d->form < DPM_FORM_NONE || d->form > DPM_FORM_SS3T ? DPM_ERR_ARG : DPM_ERR_UNSUPPORTED;
+  }
+  if (d->dev_coef != nullptr) { set_error("dpm_sde_step takes its scalars by value (dev_coef must be NULL)"); return DPM_ERR_UNSUPPORTED; }
+  if (d->raw_round != 0) { set_error("dpm_sde_step has no reference-rounding mode (raw_round must be 0)"); return DPM_ERR_UNSUPPORTED; }
+  if (noise == nullptr && offset % 4 != 0) { set_error("philox offset must be a multiple of 4"); return DPM_ERR_ARG; }
+  KParams p;
+  Needs nd;
+  int rc = build_params(d, &p, &nd, false);
+  if (rc != DPM_OK) return rc;
+  const bool vec_ok = all_aligned(p, nd) && (noise == nullptr || aligned(noise, DPM_F32));
+  rc = launch_sde_step(p, vec_ok, cn, noise, seed, offset, stream);
+  if (rc != DPM_OK) return rc;
+  return finish(stream);
+}
+
 }  // namespace dpm
 
 using namespace dpm;
@@ -274,6 +295,11 @@ int dpm_get_tuning(int* variant, int* threads, int* ctas_per_sm) {
 
 int dpm_step(const dpm_step_desc* desc, dpm_stream_t stream) {
   return step_impl(desc, static_cast<cudaStream_t>(stream));
+}
+
+int dpm_sde_step(const dpm_step_desc* desc, float noise_scale, const float* noise, uint64_t seed, uint64_t offset,
+                 dpm_stream_t stream) {
+  return sde_step_impl(desc, noise_scale, noise, seed, offset, static_cast<cudaStream_t>(stream));
 }
 
 static dpm_step_desc base_desc(void* out, const void* x, uint64_t n, int dtype, int form) {

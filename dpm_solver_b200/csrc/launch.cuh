@@ -52,6 +52,8 @@ int launch_step_direct(const KParams& p, const Tuning& t, cudaStream_t stream);
 int launch_step_scalar(const KParams& p, cudaStream_t stream);
 int launch_step_tma(const KParams& p, const Tuning& t, cudaStream_t stream);
 void philox_policy(uint64_t numel, uint32_t* grid, uint64_t* counter_offset);
+int launch_sde_step(const KParams& p, bool vec_ok, float cn, const float* noise, uint64_t seed, uint64_t offset,
+                    cudaStream_t stream);
 int launch_noise_philox(void* out, const void* x, const void* xt, const float* mask, uint64_t mask_n, uint64_t n,
                         int t_count, const float* alpha, const float* sigma, uint64_t seed, uint64_t offset,
                         int x_dtype, int out_dtype, cudaStream_t stream);

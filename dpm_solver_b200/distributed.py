@@ -17,7 +17,7 @@ import torch.distributed as dist
 
 from .plan import Coeffs
 
-_FLOAT_FIELDS = ("a", "c0", "c1", "c2", "w0", "w1", "w2", "w3", "w4")
+_FLOAT_FIELDS = ("a", "c0", "c1", "c2", "w0", "w1", "w2", "w3", "w4", "cn")
 _INT_FIELDS = ("form", "c0_on_old", "order", "r_tensor")
 _WIDTH = len(_FLOAT_FIELDS) + len(_INT_FIELDS)
 
@@ -37,7 +37,7 @@ def shard_batch(x: torch.Tensor, rank: Optional[int] = None, world: Optional[int
 
 
 def pack_plan(plan: Sequence[Coeffs]) -> torch.Tensor:
-    """[len(plan), 13] float64 table (fp32 values and small ints are exact in float64)."""
+    """[len(plan), 14] float64 table (fp32 values and small ints are exact in float64)."""
     t = torch.zeros(len(plan), _WIDTH, dtype=torch.float64)
     for i, c in enumerate(plan):
         for j, f in enumerate(_FLOAT_FIELDS):
@@ -57,7 +57,7 @@ def unpack_plan(t: torch.Tensor) -> List[Coeffs]:
 
 
 def broadcast_plan(plan: Sequence[Coeffs], src: int = 0, group=None, device=None) -> List[Coeffs]:
-    """Rank `src`'s plan on every rank: exactly one collective, len(plan)*13*8 bytes."""
+    """Rank `src`'s plan on every rank: exactly one collective, len(plan)*14*8 bytes."""
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return list(plan)
     t = pack_plan(plan)

@@ -71,6 +71,19 @@ class StepArgs:
         raise ValueError("StepArgs without tensors")
 
 
+def check_generator(generator, device) -> None:
+    """Raise ValueError unless `generator` (None = the device's default generator) draws on `device`."""
+    if generator is None:
+        return
+    if not isinstance(generator, torch.Generator):
+        raise ValueError(f"dpm_solver_b200: `generator` must be a torch.Generator, got {type(generator).__name__}")
+    gd, device = generator.device, torch.device(device)
+    g_index = gd.index if gd.index is not None or gd.type != "cuda" else torch.cuda.current_device()
+    d_index = device.index if device.index is not None or device.type != "cuda" else torch.cuda.current_device()
+    if gd.type != device.type or g_index != d_index:
+        raise ValueError(f"dpm_solver_b200: the generator is on {gd}, the tensors on {device}")
+
+
 _raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)
 if _raw_stream is None:  # older torch: go through the Stream object
     def _raw_stream(idx):
@@ -183,6 +196,12 @@ class CudaBackend:
     def step(self, a: StepArgs) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
         """Launch one fused step. Returns (m_out, out); either may be None."""
         d, keep, ref, sdt, layout = self._fill(a)
+        m_out, out = self._outputs(a, d, ref, sdt, layout)
+        self._launch(ref.device, self._lib.dpm_step, C.byref(d))
+        return m_out, out
+
+    def _outputs(self, a: StepArgs, d, ref, sdt, layout):
+        """Allocate (or check the preallocated) m_out / out / out2 of a step and point the descriptor at them."""
         m_out = out = None
         if a.n_model > 0 and (a.want_m_out or a.form == FORM_NONE):
             m_out = a.m_out if a.m_out is not None else self._new_like(ref, sdt, layout)
@@ -201,7 +220,41 @@ class CudaBackend:
                 if self._layout(a.out2) != layout:      # dense, laid out like `out` (a channels_last half of the
                     raise ValueError("dpm_solver_b200: out2 must be dense and laid out like out")   # doubled CFG batch is)
                 d.out2 = a.out2.data_ptr()
-        self._launch(ref.device, self._lib.dpm_step, C.byref(d))
+        return m_out, out
+
+    def sde_step(self, a: StepArgs, noise_scale: float, generator=None, noise: Optional[torch.Tensor] = None):
+        """One stochastic SDE-DPM-Solver step (LIN1 / DIFF2): the step `step(a)` computes plus noise_scale * z, one
+        launch (csrc/step_sde.cu). z is `torch.randn_like(x, dtype=torch.float32)` for the state of `generator` (None:
+        the default generator of the tensors' device), generated in registers, and the generator is advanced exactly
+        as that randn would advance it; or, with `noise=`, that fp32 tensor. Under CUDA-graph capture the noise is
+        drawn by torch inside the capture (replays then draw fresh noise) and read from memory; only the default
+        generator can be used there. Returns (m_out, out)."""
+        if a.form not in (FORM_LIN1, FORM_DIFF2):
+            raise ValueError("dpm_solver_b200: the SDE step serves the LIN1 and DIFF2 forms only")
+        d, keep, ref, sdt, layout = self._fill(a)
+        dev = ref.device
+        check_generator(generator, dev)
+        m_out, out = self._outputs(a, d, ref, sdt, layout)
+        seed = offset = 0
+        if noise is None and torch.cuda.is_current_stream_capturing():
+            # a (seed, offset) read on the host would be frozen into the graph: let torch draw the noise inside the
+            # capture (its default generator is capture-aware) and read it from memory
+            if generator is not None and generator is not torch.cuda.default_generators[dev.index]:
+                raise RuntimeError("dpm_solver_b200: only the default CUDA generator can draw SDE noise under "
+                                   "CUDA-graph capture")
+            noise = self._new_like(ref, torch.float32, layout).normal_()
+        if noise is not None:
+            noise = self._check(noise, "noise", dev, ref.numel(), torch.float32, layout)
+            keep.append(noise)
+            if self._layout(noise) != layout:
+                raise ValueError("dpm_solver_b200: `noise` must be dense and laid out like the inputs")
+            nptr = noise.data_ptr()
+        else:
+            nptr = None
+            with torch.cuda.device(dev):
+                seed, offset = self._philox_state(dev, ref.numel(), self._lib, generator)
+        self._launch(dev, self._lib.dpm_sde_step, C.byref(d), C.c_float(noise_scale), C.c_void_p(nptr),
+                     C.c_uint64(seed), C.c_uint64(offset))
         return m_out, out
 
     def _launch(self, device, fn, *args):

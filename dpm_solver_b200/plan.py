@@ -40,6 +40,7 @@ class Coeffs:
     order: int = 1
     r_tensor: int = 0   # SS3T: bit 0 / 1 = r1 / r2 came as tensors (matters to reference_rounding only)
     dev: Optional[torch.Tensor] = None   # scalars live in this device block instead (on-device adaptive controller)
+    cn: float = 0.0     # SDE steps: coefficient of the fresh Gaussian noise z (dpm_sde_step's noise_scale)
 
 
 def _cpu(t: torch.Tensor) -> torch.Tensor:
@@ -211,6 +212,78 @@ def multistep_plan(ns, algorithm_type, solver_type, timesteps: torch.Tensor, ord
         for k, j in enumerate(idx[3]):
             plan[j] = Coeffs(FORM_MS3, v[0][k], v[1][k], v[2][k], v[3][k], w0=v[4][k], w1=v[5][k], w2=v[6][k],
                              w3=v[7][k], order=3)
+    return plan  # type: ignore[return-value]
+
+
+# ---- stochastic multistep (SDE-DPM-Solver / SDE-DPM-Solver++) ---------------------------------
+# Step s -> t, h = lambda_t - lambda_s (s = newest buffered time), D0 = m0, D1 = (1/r0)*(m0 - m1), z ~ N(0, I):
+#   x_t = a*x + c0*D0 + c1*D1 + cn*z      (order 1: no c1 term)
+# sde-dpmsolver++ (data prediction):  a = (sigma_t/sigma_s)*exp(-h), c0 = -(alpha_t*expm1(-2h)),
+#     c1 = 0.5*c0 ('dpmsolver') | alpha_t*(expm1(-2h)/(2h) + 1) ('taylor'),  cn = sigma_t*sqrt(-expm1(-2h))
+# sde-dpmsolver (noise prediction):   a = exp(log_alpha_t - log_alpha_s), c0 = -2*sigma_t*expm1(h),
+#     c1 = -(sigma_t*expm1(h)) ('dpmsolver') | -2*sigma_t*(expm1(h)/h - 1) ('taylor'),  cn = sigma_t*sqrt(expm1(2h))
+# (the 'midpoint' and 'heun' second-order terms of the SDE solvers in Hugging Face diffusers, with expm1 in place of
+# exp - 1). Every scalar is one fp32 torch CPU op chain in the order written in _sde below.
+SDE_ALGORITHMS = ("sde-dpmsolver", "sde-dpmsolver++")
+
+
+def _sde(algorithm_type: str, solver_type: str, ms: Marginals, mt: Marginals, order: int):
+    """(a, c0, c1, cn) tensors of SDE steps ms -> mt (c1 is zero for order 1)."""
+    h = mt.lam - ms.lam
+    if algorithm_type == "sde-dpmsolver++":
+        em = torch.expm1(-2. * h)
+        a = (mt.sigma / ms.sigma) * torch.exp(-h)
+        c0 = -(mt.alpha * em)
+        if order == 1:
+            c1 = torch.zeros_like(c0)
+        elif solver_type == "dpmsolver":
+            c1 = 0.5 * c0
+        else:
+            c1 = mt.alpha * (em / (2. * h) + 1.)
+        cn = mt.sigma * torch.sqrt(-em)
+    elif algorithm_type == "sde-dpmsolver":
+        ep = torch.expm1(h)
+        a = torch.exp(mt.log_alpha - ms.log_alpha)
+        c0 = -2. * (mt.sigma * ep)
+        if order == 1:
+            c1 = torch.zeros_like(c0)
+        elif solver_type == "dpmsolver":
+            c1 = -(mt.sigma * ep)
+        else:
+            c1 = -2. * (mt.sigma * (ep / h - 1.))
+        cn = mt.sigma * torch.sqrt(torch.expm1(2. * h))
+    else:
+        raise ValueError("not an SDE algorithm_type: {!r}".format(algorithm_type))
+    return a, c0, c1, cn
+
+
+def sde_multistep_plan(ns, algorithm_type, solver_type, timesteps: torch.Tensor, order: int,
+                       lower_order_final: bool, marginals: Optional[Marginals] = None) -> List[Coeffs]:
+    """Coefficients of every step of a stochastic multistep run (orders 1 and 2; the order schedule of
+    multistep_orders); plan[i] moves timesteps[i] -> [i+1]. Order 1 steps are LIN1, order 2 steps DIFF2 with
+    w0 = 1/r0 exactly as in multistep_plan."""
+    if order not in (1, 2):
+        raise ValueError("{} is served by multistep orders 1 and 2, got order {}".format(algorithm_type, order))
+    ts = _cpu(timesteps)
+    steps = ts.numel() - 1
+    M = marginals if marginals is not None else Marginals(ns, ts)
+    orders = multistep_orders(steps, order, lower_order_final)
+    plan: List[Optional[Coeffs]] = [None] * steps
+    for p in (1, 2):
+        idx = [i for i, o in enumerate(orders) if o == p]
+        if not idx:
+            continue
+        i = torch.tensor(idx)
+        a, c0, c1, cn = (v.reshape(-1).tolist() for v in _sde(algorithm_type, solver_type, M[i], M[i + 1], p))
+        if p == 1:
+            for k, j in enumerate(idx):
+                plan[j] = Coeffs(FORM_LIN1, a[k], c0[k], order=1, cn=cn[k])
+        else:
+            h_0 = M[i].lam - M[i - 1].lam
+            h = M[i + 1].lam - M[i].lam
+            w0 = (1. / (h_0 / h)).reshape(-1).tolist()      # 1/r0, as multistep_plan
+            for k, j in enumerate(idx):
+                plan[j] = Coeffs(FORM_DIFF2, a[k], c0[k], c1[k], w0=w0[k], order=2, cn=cn[k])
     return plan  # type: ignore[return-value]
 
 

@@ -239,8 +239,10 @@ class DPM_Solver:
             # the reference would promote x and every update to that dtype; there are no fp64 kernels
             raise TypeError("dpm_solver_b200 computes in fp32: NoiseScheduleVP(dtype={}) is not supported "
                             "by DPM_Solver".format(tables.dtype))
-        assert algorithm_type in ["dpmsolver", "dpmsolver++"]
+        assert algorithm_type in ["dpmsolver", "dpmsolver++"] + list(P.SDE_ALGORITHMS)
         self.algorithm_type = algorithm_type
+        if reference_rounding and algorithm_type in P.SDE_ALGORITHMS:
+            raise ValueError("reference_rounding=True is not available for algorithm_type={!r}".format(algorithm_type))
         if correcting_x0_fn == "dynamic_thresholding":
             self.correcting_x0_fn = self.dynamic_thresholding_fn
             self._dynamic_thresholding = True
@@ -296,7 +298,18 @@ class DPM_Solver:
     # -- small helpers ------------------------------------------------------------------------
     @property
     def _pp(self) -> bool:
-        return self.algorithm_type == "dpmsolver++"
+        """The buffered model value is x0 (data prediction)."""
+        return self.algorithm_type in ("dpmsolver++", "sde-dpmsolver++")
+
+    @property
+    def _sde(self) -> bool:
+        return self.algorithm_type in P.SDE_ALGORITHMS
+
+    def _no_sde(self, what: str) -> None:
+        """The stochastic solvers exist as multistep sample() runs only; never run them silently as the ODE."""
+        if self._sde:
+            raise ValueError("{} is not available for algorithm_type={!r}: the SDE solvers are served by "
+                             "sample(method='multistep', order=1 or 2)".format(what, self.algorithm_type))
 
     def _sdtype(self, x) -> torch.dtype:
         if self.state_dtype is not None:
@@ -558,7 +571,7 @@ class DPM_Solver:
         dup = self._dup_target(x) if dup_out else None
         if dup is not None:
             a.out, a.out2 = dup[1], dup[2]
-        m_new, x_next = be.step(a)
+        m_new, x_next = self._launch(a, co)
         if dup is not None:
             self._xin_pair = (x_next, dup[0])
         if pkey is not None and not a.per_sample:
@@ -601,10 +614,18 @@ class DPM_Solver:
         a = StepArgs(n_model=0, m0=self._state_like(m0, x.dtype), state_dtype=x.dtype, raw_round=rr)
         self._fill_update(a, co, x, None if m1 is None else self._state_like(m1, x.dtype),
                           None if m2 is None else self._state_like(m2, x.dtype))
-        out = ops.backend().step(a)[1]
+        out = self._launch(a, co)[1]
         if pkey is not None and not rr:
             self._remember(pkey, a)
         return out
+
+    def _launch(self, a: StepArgs, co: P.Coeffs):
+        """One update launch: the ODE step, or for the SDE algorithms the same step plus co.cn * (fresh noise drawn
+        from the generator of the sample() call in flight)."""
+        be = ops.backend()
+        if self._sde:
+            return be.sde_step(a, co.cn, generator=self.__dict__.get("_generator"))
+        return be.step(a)
 
     # -- reference API: model functions ---------------------------------------------------------
     def dynamic_thresholding_fn(self, x0, t):
@@ -670,6 +691,7 @@ class DPM_Solver:
     # -- reference API: single updates (direct-call path; scalars computed per call) -------------
     def dpm_solver_first_update(self, x, s, t, model_s=None, return_intermediate=False):
         """DPM-Solver-1 / DDIM step s -> t (:547-592)."""
+        self._no_sde("dpm_solver_first_update")
         x = self._state(x)
         co = P.first_update_coeffs(self.noise_schedule, self.algorithm_type, s, t)
         if model_s is None:
@@ -687,6 +709,7 @@ class DPM_Solver:
     def singlestep_dpm_solver_second_update(self, x, s, t, r1=0.5, model_s=None, return_intermediate=False,
                                             solver_type='dpmsolver'):
         """Singlestep DPM-Solver-2 s -> t (:594-673)."""
+        self._no_sde("singlestep_dpm_solver_second_update")
         if solver_type not in ['dpmsolver', 'taylor']:
             raise ValueError("'solver_type' must be either 'dpmsolver' or 'taylor', got {}".format(solver_type))
         sp = P.singlestep_second(self.noise_schedule, self.algorithm_type, solver_type, s, t, r1)
@@ -698,6 +721,7 @@ class DPM_Solver:
     def singlestep_dpm_solver_third_update(self, x, s, t, r1=1. / 3., r2=2. / 3., model_s=None, model_s1=None,
                                            return_intermediate=False, solver_type='dpmsolver'):
         """Singlestep DPM-Solver-3 s -> t (:675-794)."""
+        self._no_sde("singlestep_dpm_solver_third_update")
         if solver_type not in ['dpmsolver', 'taylor']:
             raise ValueError("'solver_type' must be either 'dpmsolver' or 'taylor', got {}".format(solver_type))
         sp = P.singlestep_third(self.noise_schedule, self.algorithm_type, solver_type, s, t, r1, r2)
@@ -752,6 +776,7 @@ class DPM_Solver:
 
     def multistep_dpm_solver_second_update(self, x, model_prev_list, t_prev_list, t, solver_type="dpmsolver"):
         """Multistep DPM-Solver-2 (:796-852)."""
+        self._no_sde("multistep_dpm_solver_second_update")
         if solver_type not in ['dpmsolver', 'taylor']:
             raise ValueError("'solver_type' must be either 'dpmsolver' or 'taylor', got {}".format(solver_type))
         co = P.multistep_coeffs(self.noise_schedule, self.algorithm_type, solver_type, 2, t_prev_list, t)
@@ -759,6 +784,7 @@ class DPM_Solver:
 
     def multistep_dpm_solver_third_update(self, x, model_prev_list, t_prev_list, t, solver_type='dpmsolver'):
         """Multistep DPM-Solver-3 (:854-904); needs exactly three buffered values."""
+        self._no_sde("multistep_dpm_solver_third_update")
         model_prev_2, model_prev_1, model_prev_0 = model_prev_list
         t_prev_2, t_prev_1, t_prev_0 = t_prev_list
         co = P.multistep_coeffs(self.noise_schedule, self.algorithm_type, solver_type, 3,
@@ -768,6 +794,7 @@ class DPM_Solver:
     def singlestep_dpm_solver_update(self, x, s, t, order, return_intermediate=False, solver_type='dpmsolver',
                                      r1=None, r2=None):
         """Order dispatch (:906-930)."""
+        self._no_sde("singlestep_dpm_solver_update")
         if order == 1:
             return self.dpm_solver_first_update(x, s, t, return_intermediate=return_intermediate)
         elif order == 2:
@@ -781,6 +808,7 @@ class DPM_Solver:
 
     def multistep_dpm_solver_update(self, x, model_prev_list, t_prev_list, t, order, solver_type='dpmsolver'):
         """Order dispatch (:932-954)."""
+        self._no_sde("multistep_dpm_solver_update")
         if order == 1:
             return self.dpm_solver_first_update(x, t_prev_list[-1], t, model_s=model_prev_list[-1])
         elif order == 2:
@@ -795,6 +823,7 @@ class DPM_Solver:
                             t_err=1e-5, solver_type='dpmsolver'):
         """Adaptive step size DPM-Solver-12 / -23 (:956-1010). Updates and the error estimate run on
         the fused kernels; the step-size controller is the reference's host logic."""
+        self._no_sde("the adaptive solver")
         ns = self.noise_schedule
         x = self._state(x)
         device = x.device
@@ -949,6 +978,7 @@ class DPM_Solver:
                 method='multistep', lower_order_final=True, denoise_to_zero=False, solver_type='dpmsolver',
                 atol=0.0078, rtol=0.05, return_intermediate=False):
         """Invert `x` from t_start (default 1/N) to t_end (default T) (:1032-1045)."""
+        self._no_sde("inverse()")
         t_0 = 1. / self.noise_schedule.total_N if t_start is None else t_start
         t_T = self.noise_schedule.T if t_end is None else t_end
         assert t_0 > 0 and t_T > 0, "Time range needs to be greater than 0. For discrete-time DPMs, it needs to be in [1 / N, 1], where N is the length of betas array"
@@ -970,6 +1000,11 @@ class DPM_Solver:
             raise ValueError("the adaptive solver decides on the host every iteration; it cannot be captured")
         if sample_kwargs.get("return_intermediate"):
             raise ValueError("capture() returns the final sample only")
+        gen = sample_kwargs.get("generator")
+        if self._sde and gen is not None and gen is not torch.cuda.default_generators[torch.device(gen.device).index or 0]:
+            # the noise of a captured SDE run is drawn inside the graph, which only the default generator follows
+            raise ValueError("capture() of algorithm_type={!r} draws its noise from the default CUDA generator; "
+                             "pass generator=None".format(self.algorithm_type))
         x_static = self._state(x_example).clone()
         self.sample(x_static, **sample_kwargs)                       # builds and caches plan + tables
         graph = torch.cuda.CUDAGraph()
@@ -992,8 +1027,12 @@ class DPM_Solver:
     # -- sample (:1047-1245) ---------------------------------------------------------------------
     def sample(self, x, steps=20, t_start=None, t_end=None, order=2, skip_type='time_uniform',
                method='multistep', lower_order_final=True, denoise_to_zero=False, solver_type='dpmsolver',
-               atol=0.0078, rtol=0.05, return_intermediate=False):
-        """Integrate the diffusion ODE from t_start to t_end; arguments as in the reference."""
+               atol=0.0078, rtol=0.05, return_intermediate=False, generator=None):
+        """Integrate the diffusion ODE from t_start to t_end; arguments as in the reference.
+
+        For algorithm_type "sde-dpmsolver++" / "sde-dpmsolver" (method='multistep', order 1 or 2) the diffusion SDE is
+        integrated instead: every step adds fresh Gaussian noise, drawn in the step kernel from `generator` (a
+        torch.Generator on x's device; None = that device's default generator). The ODE algorithms ignore it."""
         t_0 = 1. / self.noise_schedule.total_N if t_end is None else t_end
         t_T = self.noise_schedule.T if t_start is None else t_start
         assert t_0 > 0 and t_T > 0, "Time range needs to be greater than 0. For discrete-time DPMs, it needs to be in [1 / N, 1], where N is the length of betas array"
@@ -1002,12 +1041,21 @@ class DPM_Solver:
         if self.correcting_xt_fn is not None:
             assert method in ['multistep', 'singlestep', 'singlestep_fixed'], "Cannot use adaptive solver when correcting_xt_fn is not None"
         device = x.device
+        if self._sde:
+            if method != 'multistep':
+                self._no_sde("method={!r}".format(method))
+            if order not in (1, 2):
+                raise ValueError("algorithm_type={!r} is served by multistep orders 1 and 2, got order {}".format(
+                    self.algorithm_type, order))
+            ops.check_generator(generator, device)
+        self._generator = generator if self._sde else None
         intermediates = []
         ns = self.noise_schedule
         self._xin_pair = None
         self._rr_run = 0
         # prepared launches: the CUDA executor, no python-side x0 hook, no 16-bit reference-rounding mode
-        self._prep_on = (hasattr(ops.backend(), "prepare") and not self.reference_rounding
+        # (not for the SDE algorithms: a frozen descriptor launches dpm_step, which adds no noise)
+        self._prep_on = (hasattr(ops.backend(), "prepare") and not self.reference_rounding and not self._sde
                          and (self.correcting_x0_fn is None or self._dynamic_thresholding))
         with torch.no_grad():
             x = self._state(x)
@@ -1028,8 +1076,8 @@ class DPM_Solver:
                     ts = self.get_time_steps(skip_type=skip_type, t_T=t_T, t_0=t_0, N=steps, device='cpu')
                     assert ts.shape[0] - 1 == steps
                     marg = P.Marginals(ns, ts)
-                    plan = P.multistep_plan(ns, self.algorithm_type, solver_type, ts, order, lower_order_final,
-                                            marginals=marg)
+                    mk = P.sde_multistep_plan if self._sde else P.multistep_plan
+                    plan = mk(ns, self.algorithm_type, solver_type, ts, order, lower_order_final, marginals=marg)
                     # (alpha_t, sigma_t) per grid point: scalars of the eps->x0 / parameterisation step
                     return ts, plan, list(zip(marg.alpha.tolist(), marg.sigma.tolist()))
 
@@ -1140,6 +1188,7 @@ class DPM_Solver:
                 if return_intermediate:
                     intermediates.append(x)
         self._net_input = None
+        self._generator = None
         if return_intermediate:
             return x, intermediates
         else:

@@ -219,6 +219,20 @@ DPM_API int dpm_add_noise_philox(void* xt, const void* x, uint64_t n, int t_coun
                                  const float* sigma_t, uint64_t seed, uint64_t offset, int x_dtype, int out_dtype,
                                  dpm_stream_t stream);
 
+/* One stochastic SDE-DPM-Solver(++) multistep step (orders 1 and 2): the step dpm_step(desc) computes, plus one
+ * separately rounded noise term,
+ *   out = ((a*x + c0*NEW) + c1*D) + noise_scale*z        (form LIN1: out = (a*x + c0*NEW) + noise_scale*z)
+ * with every other field of desc read as dpm_step reads it (n_model 0/1/2, param, CFG, predict_x0, thr, m_out, out2).
+ * z is element i, in storage order, of
+ *   noise != NULL: the fp32 array noise[n];
+ *   noise == NULL: torch.randn(n) drawn from a torch CUDA generator in state (seed, offset), generated in registers
+ *                  with the virtual grid of dpm_philox_policy(desc->n); the caller advances the generator's offset
+ *                  by that policy's counter_offset. offset must be a multiple of 4.
+ * Only DPM_FORM_LIN1 and DPM_FORM_DIFF2 are served, with the scalars by value: another form, dev_coef != NULL or
+ * raw_round != 0 returns DPM_ERR_UNSUPPORTED. */
+DPM_API int dpm_sde_step(const dpm_step_desc* desc, float noise_scale, const float* noise, uint64_t seed,
+                         uint64_t offset, dpm_stream_t stream);
+
 /* DiffEdit corrector (examples/stable-diffusion/scripts/diffedit_inpaint.ipynb corrector_fn + sampler.py:92-96):
  *   out = x*mask + (1 - mask)*(alpha_t*x0 + sigma_t*randn_like(x0)),  one launch, noise in registers.
  * mask: fp32, mask_n elements, broadcast over the leading dimensions of x (n % mask_n == 0). */
